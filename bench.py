@@ -16,9 +16,15 @@ every launch reads cold (HBM-resident, not L2-resident) data.
 `e2e` = the same metric through the reference-facing class (MultiDiffusion.kdiff_forward, identity
 denoiser) with the step's latent copied from pinned host memory and the blended result copied back.
 
-`--impl reference` / `cpu_baseline` = the UNMODIFIED reference's `sample_one_step` under the stub host where
-/root/reference exists (`kind: "reference"`), else its op-for-op restatement (oracle/blend.py, bit-identical to the
-reference; `kind: "port"`), on this box's host cores at the thread count that runs it fastest, identity denoiser.
+`--impl reference` / `cpu_baseline` = the op-for-op restatement of the reference's `sample_one_step` (oracle/blend.py,
+bit-identical to the reference; `kind: "port"`) on the host cores at the thread count that runs it fastest, identity
+denoiser.
+
+`--dump-outputs DIR` (single GPU) writes what the last timed step computed, as float32 .npy files: cfg2 / cfg3 the tile
+batch td_scatter_tiles hands the UNet (`tiles.npy`) and the blended latent (`latent.npy`); cfg4 the decoded image at 2^21
+pixel positions drawn with a fixed seed (`image_sample.npy` [3, 2^21], positions y * W + x in `image_sample_index.npy`,
+float64); cfg5 the step's latent (`latent.npy`).  The inputs are seeded, so two builds run with the same arguments can be
+compared output for output.  `--steps` is used exactly as given.
 
 Other BASELINE configs (same JSON contract, DESIGN.md section 6):
     --config cfg3   Mixture of Diffusers step (td_blend_mixture heads the roofline object)
@@ -120,28 +126,16 @@ class ClockSampler:
 
 # ----------------------------------------------------------------------------- CPU arm
 def cpu_reference_step_fn(method: str = "md"):
-    """One sampler step of the reference's PyTorch tile path on the host cores, identity denoiser.
-
-    When the reference tree is present (build container) this is the UNMODIFIED reference:
-    `MultiDiffusion.sample_one_step` imported through oracle/ref_shim.py (kind "reference").  The GPU box has no
-    /root/reference; there it is the oracle restatement, which executes the reference's exact op sequence
-    (`x_buffer[slicer] += tile` in the latent dtype, `torch.where(weights > 1, x_buffer / weights, x_buffer)`;
-    oracle/blend.py, bit-identical outputs, same speed within noise: 4.2 vs 4.2 ms here) -- kind "port"."""
-    from oracle import blend, ref_shim, synth, tiling
+    """One sampler step of the reference's PyTorch tile path on the host cores, identity denoiser: the oracle
+    restatement, which executes the reference's exact op sequence (`x_buffer[slicer] += tile` in the latent dtype,
+    `torch.where(weights > 1, x_buffer / weights, x_buffer)`; oracle/blend.py, bit-identical outputs, same speed within
+    noise as the unmodified reference: 4.2 vs 4.2 ms on one host) -- kind "port"."""
+    from oracle import blend, synth, tiling
     c = CFG
     x = synth.latent(0, (c["N"], c["C"], c["H"], c["W"]), torch.float16)
     if method == "mod":      # Mixture of Diffusers: op-for-op restatement (mixtureofdiffusers.py:61-179 grid part)
         plan = tiling.GridPlan(c["W"], c["H"], c["tile"], c["tile"], c["overlap"], c["tile_bs"], True)
         return (lambda: blend.mixture_step(x, plan.batched_bboxes, plan.tile_weights, plan.rescale_factor, lambda t, bb: t)), "port"
-    if ref_shim.available():
-        ref = ref_shim.load()
-        p = ref_shim.make_p(c["W"] * 8, c["H"] * 8)
-        sampler = ref_shim.make_kdiff_sampler(lambda *a, **k: None)
-        d = ref.multidiffusion.MultiDiffusion(p, sampler)
-        d.init_grid_bbox(c["tile"], c["tile"], c["overlap"], c["tile_bs"])
-        d.init_done()
-        d.pbar.disable = True
-        return (lambda: d.sample_one_step(x, None, lambda t, bb: t, None)), "reference"
     plan = tiling.GridPlan(c["W"], c["H"], c["tile"], c["tile"], c["overlap"], c["tile_bs"], False)
     return (lambda: blend.multidiffusion_step(x, plan.batched_bboxes, plan.weights, lambda t, bb: t)), "port"
 
@@ -223,8 +217,7 @@ def reference_arm(args, rank):
         "vs_baseline": None, "dtype": "f16", "data": "synthetic", "config": workload_config(),
         "cpu_baseline": {"value": v, "unit": "MP/s", "cores": threads, "kind": kind,
                          "sample": f"{done} sampler steps of cfg2 (scatter+blend+normalise, identity denoiser), torch CPU, "
-                                   + ("unmodified reference sample_one_step" if kind == "reference" else
-                                      "op-for-op restatement of the reference's sample_one_step (no /root/reference on this box)")},
+                                   "op-for-op restatement of the reference's sample_one_step"},
         "e2e": {"value": v, "unit": "MP/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
     }
@@ -448,6 +441,11 @@ class Workload:
         c = self.cabi
         c.check(c.lib.td_debug_launch_empty(1024, 128, self.stream))
 
+    def outputs(self, s):
+        """What a step on buffer set `s` hands on: the tile batch for the UNet and the blended latent (fp32 for
+        MultiDiffusion, the latent dtype for Mixture of Diffusers)."""
+        return {"tiles": self.tiles_in[s], "latent": self._mod[2][s] if self.method == "mod" else self.x_out[s]}
+
     def step(self, i):
         s = i % self.nsets
         self.scatter(s)
@@ -514,6 +512,14 @@ def timed_graph_loop(fn_step, steps, stream, chunk=1024):
     return replay
 
 
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: each tensor of `arrays` as <out_dir>/<name>.npy, float64 kept, everything else as float32."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), (t if t.dtype == torch.float64 else t.float()).cpu().numpy())
+
+
 def event_time_ms(fn, stream):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     torch.cuda.synchronize()
@@ -531,8 +537,8 @@ def gpu_arm(args, rank, world, local_rank):
         torch.distributed.init_process_group("nccl", device_id=dev)
     peak, peak_src = load_peaks()
     nsets = args.buffer_sets
-    if world > 1:   # peer exchange is double-buffered by step parity: keep every launch group even
-        args.steps += args.steps & 1
+    torch.manual_seed(0)      # the synthetic tile outputs are the same in every run
+    if world > 1:   # peer exchange is double-buffered by step parity: keep every launch group even (odd --steps refused in main)
         args.warmup = max(args.warmup, 4) + (max(args.warmup, 4) & 1)
     wl = Workload(dev, rank, world, nsets, args.exchange)
     mod = args.config == "cfg3"
@@ -570,6 +576,8 @@ def gpu_arm(args, rank, world, local_rank):
             torch.distributed.all_reduce(t, op=torch.distributed.ReduceOp.MAX)
         ms = float(t.item())
         sec_per_step = ms / 1e3 / args.steps
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, wl.outputs((args.steps - 1) % nsets))
 
         # --- per-kernel duration for the roofline (same buffers, same stream, CUDA events) -------------
         roof = None
@@ -660,10 +668,8 @@ def gpu_arm(args, rank, world, local_rank):
             "roofline": roof,
             "cpu_baseline": {"value": mp_per_s(cpu_dt), "unit": "MP/s", "cores": cpu_threads, "kind": cpu_kind,
                              "ms_per_step": cpu_dt * 1e3,
-                             "sample": f"{cpu_done} sampler steps of the same workload ("
-                                       + ("unmodified reference sample_one_step" if cpu_kind == "reference" else
-                                          "op-for-op restatement of the reference's sample_one_step") +
-                                       f", identity denoiser, torch CPU, {cpu_threads} threads)",
+                             "sample": f"{cpu_done} sampler steps of the same workload (op-for-op restatement of the "
+                                       f"reference's sample_one_step, identity denoiser, torch CPU, {cpu_threads} threads)",
                              "eager_cuda": eager_cuda_baseline("mod" if mod else "md") if world == 1 and args.cpu_budget > 1.0 else None},
             "impl": "b200",
         }
@@ -1021,17 +1027,26 @@ def vae_arm(args, rank, world, local_rank):
     mp = (lat * 8) ** 2 / 1e6
     stream = torch.cuda.current_stream(dev)
     sampler = ClockSampler(local_rank).start() if rank == 0 else None
-    steps, warm = max(1, min(args.steps, 5)), max(1, min(args.warmup, 2))
+    steps, warm = args.steps, max(1, min(args.warmup, 2))
     for _ in range(warm):
         y = hook(z)
     torch.cuda.synchronize()
     if world > 1:
         torch.distributed.barrier()
-    ms = event_time_ms(lambda: [hook(z) for _ in range(steps)], stream)
+    last = {}
+
+    def timed():
+        for _ in range(steps):
+            last["y"] = hook(z)
+    ms = event_time_ms(timed, stream)
     t = torch.tensor([ms], device=dev)
     if world > 1:
         torch.distributed.all_reduce(t, op=torch.distributed.ReduceOp.MAX)
     sec = float(t.item()) / 1e3 / steps
+    if args.dump_outputs:      # the 8192^2 image is 805 MB in fp32: a fixed, seeded sample of 2^21 pixels, with their positions
+        img = last["y"].reshape(last["y"].shape[1], -1)
+        idx = torch.randint(img.shape[1], (min(1 << 21, img.shape[1]),), generator=torch.Generator().manual_seed(0))
+        dump_outputs(args.dump_outputs, {"image_sample": img[:, idx.to(dev)], "image_sample_index": idx.double()})
 
     def e2e_step():
         zd = z_host.to(dev, non_blocking=True)
@@ -1104,10 +1119,10 @@ def vae_arm(args, rank, world, local_rank):
         torch.distributed.barrier()
 
 
-def vae_cpu_baseline(budget_s: float):
+def vae_cpu_baseline(budget_s: float, steps: int = 1):
     """The reference's tiled VAE algorithm on the host cores (oracle restatement, fp32 torch CPU) on a bounded sample:
-    a 48 / 64 / 96-pixel latent (384^2 .. 768^2 px image) decoded in 4 tiles, fast mode; thread count and sample size are
-    chosen from a short probe so that the leg stays within about 2.5 x --cpu-budget seconds."""
+    `steps` decodes of a 48 / 64 / 96-pixel latent (384^2 .. 768^2 px image) in 4 tiles, fast mode; thread count and sample
+    size are chosen from a short probe so that one decode stays within about 2.5 x --cpu-budget seconds."""
     if budget_s <= 1.0:      # measurement runs that only want the GPU numbers
         return {"value": None, "unit": "MP/s", "cores": 0, "kind": "port", "seconds": 0.0, "sample": "skipped (--cpu-budget <= 1)"}
     from oracle import ldm_vae, vae
@@ -1130,19 +1145,20 @@ def vae_cpu_baseline(budget_s: float):
     z = torch.randn((1, 4, L, L), generator=torch.Generator().manual_seed(7))
     t0 = time.perf_counter()
     with torch.no_grad():
-        vae.vae_hook_call(net, z, L // 2, True, True, False)
+        for _ in range(steps):
+            vae.vae_hook_call(net, z, L // 2, True, True, False)
     dt = time.perf_counter() - t0
-    return {"value": (L * 8) ** 2 / 1e6 / dt, "unit": "MP/s", "cores": torch.get_num_threads(), "kind": "port", "seconds": dt,
-            "sample": f"one tiled decode of a {L}x{L} latent ({L * 8}x{L * 8} px, decoder tile {L // 2}, fast mode: 4 tiles + estimator pass), "
+    return {"value": (L * 8) ** 2 / 1e6 / (dt / steps), "unit": "MP/s", "cores": torch.get_num_threads(), "kind": "port", "seconds": dt,
+            "steps": steps, "sample": f"{steps} tiled decode(s) of a {L}x{L} latent ({L * 8}x{L * 8} px, decoder tile {L // 2}, fast mode: 4 tiles + estimator pass), "
                       "oracle restatement of scripts/tilevae.py on torch CPU fp32"}
 
 
 def vae_reference_arm(args, rank):
     if rank != 0:
         return
-    cpu = vae_cpu_baseline(args.cpu_budget)
-    line = {"impl": "reference", "metric": VAE_METRIC, "value": cpu["value"], "unit": "MP/s", "n_gpus": args.gpus, "steps": 1, "warmup": 0,
-            "ms_per_step": cpu["seconds"] * 1e3, "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f32",
+    cpu = vae_cpu_baseline(args.cpu_budget, args.steps or 1)
+    line = {"impl": "reference", "metric": VAE_METRIC, "value": cpu["value"], "unit": "MP/s", "n_gpus": args.gpus,
+            "steps": cpu.get("steps", 0), "warmup": 0, "ms_per_step": cpu["seconds"] * 1e3 / max(cpu.get("steps", 0), 1), "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f32",
             "data": "synthetic", "config": {"workload": cpu["sample"]}, "cpu_baseline": cpu,
             "e2e": {"value": cpu["value"], "unit": "MP/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}, "gpu_launches": 0}
     print(json.dumps(line), flush=True)
@@ -1200,7 +1216,7 @@ def demofusion_arm(args, rank, world, local_rank):
     sigma = torch.ones(N, device=dev)
     cond = {"c_crossattn": [torch.zeros(N, 77, 2048, device=dev, dtype=torch.float16)], "c_concat": [torch.zeros(N, 5, 1, 1, device=dev, dtype=torch.float16)]}
     stream = torch.cuda.current_stream(dev)
-    steps, warm = max(1, min(args.steps, 200)), max(3, min(args.warmup, 10))
+    steps, warm = args.steps, max(3, min(args.warmup, 10))
     sampler = ClockSampler(local_rank).start() if rank == 0 else None
     for _ in range(warm):
         y = d.sample_one_step(x, sigma, cond)
@@ -1208,12 +1224,19 @@ def demofusion_arm(args, rank, world, local_rank):
     if world > 1:
         torch.distributed.barrier()
     calls[0] = 0
-    ms = event_time_ms(lambda: [d.sample_one_step(x, sigma, cond) for _ in range(steps)], stream)
+    last = {}
+
+    def timed():
+        for _ in range(steps):
+            last["y"] = d.sample_one_step(x, sigma, cond)
+    ms = event_time_ms(timed, stream)
     unet_calls = calls[0] // steps
     t = torch.tensor([ms], device=dev)
     if world > 1:
         torch.distributed.all_reduce(t, op=torch.distributed.ReduceOp.MAX)
     sec = float(t.item()) / 1e3 / steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"latent": last["y"]})
 
     def e2e_step():
         xd = x_host.to(dev, non_blocking=True)
@@ -1287,8 +1310,9 @@ def demofusion_arm(args, rank, world, local_rank):
         torch.distributed.barrier()
 
 
-def demofusion_cpu_baseline(budget_s: float):
-    """The reference's DemoFusion step (oracle restatement, torch CPU) on the cfg5 latent in fp32, identity UNet stand-in."""
+def demofusion_cpu_baseline(budget_s: float, steps: int = None):
+    """The reference's DemoFusion step (oracle restatement, torch CPU) on the cfg5 latent in fp32, identity UNet stand-in:
+    `steps` steps, or as many as fit in `budget_s` seconds (at most 50) when `steps` is None."""
     if budget_s <= 1.0:
         return {"value": None, "unit": "MP/s", "cores": 0, "kind": "port", "seconds": 0.0, "sample": "skipped (--cpu-budget <= 1)"}
     from oracle import demofusion as odf
@@ -1314,19 +1338,19 @@ def demofusion_cpu_baseline(budget_s: float):
         while True:
             one()
             n += 1
-            if time.perf_counter() - t0 > budget_s or n >= 50:
+            if n == steps or steps is None and (time.perf_counter() - t0 > budget_s or n >= 50):
                 break
     dt = (time.perf_counter() - t0) / n
     return {"value": (L * 8) ** 2 / 1e6 / dt, "unit": "MP/s", "cores": torch.get_num_threads(), "kind": "port", "seconds": dt * n,
-            "sample": f"{n} whole cfg5 steps (latent [2,4,{L},{L}], fp32 on the host cores), oracle restatement of tile_methods/demofusion.py:219-324"}
+            "steps": n, "sample": f"{n} whole cfg5 steps (latent [2,4,{L},{L}], fp32 on the host cores), oracle restatement of tile_methods/demofusion.py:219-324"}
 
 
 def demofusion_reference_arm(args, rank):
     if rank != 0:
         return
-    cpu = demofusion_cpu_baseline(max(args.cpu_budget, 5.0))
-    line = {"impl": "reference", "metric": DEMO_METRIC, "value": cpu["value"], "unit": "MP/s", "n_gpus": args.gpus, "steps": 1, "warmup": 0,
-            "ms_per_step": (DEMO["lat"] * 8) ** 2 / 1e6 / cpu["value"] * 1e3, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
+    cpu = demofusion_cpu_baseline(max(args.cpu_budget, 5.0), args.steps)
+    line = {"impl": "reference", "metric": DEMO_METRIC, "value": cpu["value"], "unit": "MP/s", "n_gpus": args.gpus, "steps": cpu["steps"],
+            "warmup": 0, "ms_per_step": cpu["seconds"] / cpu["steps"] * 1e3, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
             "dtype": "f32", "data": "synthetic", "config": {"workload": cpu["sample"]}, "cpu_baseline": cpu,
             "e2e": {"value": cpu["value"], "unit": "MP/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}, "gpu_launches": 0}
     print(json.dumps(line), flush=True)
@@ -1335,7 +1359,8 @@ def demofusion_reference_arm(args, rank):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=2000)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps, used exactly as given (default: 2000 for cfg2 / cfg3, 5 "
+                    "decodes for cfg4, 200 for cfg5; the cfg4 / cfg5 reference arms: 1 decode / as many steps as --cpu-budget allows)")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--buffer-sets", type=int, default=8)
@@ -1351,10 +1376,21 @@ def main():
                     "(default, the headline), cfg3 = Mixture of Diffusers hot path, cfg4 = tiled VAE decode only, cfg5 = DemoFusion step")
     ap.add_argument("--vae-latent", type=int, default=1024, help="cfg4: latent edge (1024 -> 8192^2 image)")
     ap.add_argument("--vae-slow", action="store_true", help="cfg4: slow mode (GroupNorm statistics merged over all tiles at every site)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="single GPU: write what the last timed step computed to DIR/<name>.npy "
+                    "(float32; cfg4: a fixed, seeded sample of the image)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.steps is None:
+        if args.impl == "b200" or args.config in ("cfg2", "cfg3"):
+            args.steps = {"cfg2": 2000, "cfg3": 2000, "cfg4": 5, "cfg5": 200}[args.config]
+    elif args.steps < 1:
+        ap.error("--steps must be at least 1")
+    elif args.steps & 1 and world > 1 and args.impl == "b200" and args.config in ("cfg2", "cfg3") and args.exchange != "strip":
+        ap.error("--steps must be even for the peer / nccl exchange (its buffers alternate by step parity)")
+    if args.dump_outputs and (args.impl != "b200" or world > 1):
+        ap.error("--dump-outputs is for the single-GPU runs of the GPU arm")
     if args.impl == "reference":
         {"cfg4": vae_reference_arm, "cfg5": demofusion_reference_arm}.get(args.config, reference_arm)(args, rank)
         return

@@ -12,7 +12,6 @@ CUDA path, never the product:
 Pinning: the reference ships no tests or golden vectors (SURVEY.md section 4), so the
 oracle is pinned against OUTPUTS OF THE REFERENCE ITSELF, produced by importing the
 unmodified reference under the stub host in `oracle/ref_shim.py`
-(`oracle/make_golden.py` -> `tests/golden/*.npz`, committed together with the
-generating script) and -- when `/root/reference` is present -- by calling the
-reference live in `tests/test_oracle_vs_reference.py`.
+(`oracle/make_golden.py`, `oracle/make_reference_traces.py` -> `tests/golden/*.npz`,
+committed together with the generating scripts).
 """

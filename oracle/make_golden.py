@@ -1,8 +1,8 @@
 """TEST INFRASTRUCTURE -- generate tests/golden/*.npz FROM THE UNMODIFIED REFERENCE.
 
-Run in the build container only (needs /root/reference):
+Needs a checkout of the original extension:
 
-    python -m oracle.make_golden
+    TD_REFERENCE_ROOT=<checkout of the original extension> python -m oracle.make_golden
 
 Every array below is an output of the reference's own code
 (tile_utils/utils.py, tile_methods/{multidiffusion,mixtureofdiffusers}.py,
@@ -284,7 +284,7 @@ def run_reference_step(ref, method: str, x: torch.Tensor, W, H, tw, th, ov, bs):
 
 def main():
     if not ref_shim.available():
-        sys.exit("reference tree not present; goldens can only be generated in the build container")
+        sys.exit("reference tree not found: set TD_REFERENCE_ROOT to a checkout of the original extension")
     os.makedirs(GOLDEN_DIR, exist_ok=True)
     ref = ref_shim.load()
     torch.set_num_threads(1)

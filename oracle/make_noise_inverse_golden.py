@@ -1,9 +1,9 @@
-"""TEST INFRASTRUCTURE -- fixture of tiled noise inversion from the UNMODIFIED reference (build container only).
+"""TEST INFRASTRUCTURE -- fixture of tiled noise inversion from the UNMODIFIED reference.
 
 Runs the reference's `sample_img2img` replacement (tile_methods/abstractdiffusion.py:604-742 + multidiffusion.py:220-243)
 on CPU under oracle/ref_shim.py for the job defined in tests/noise_inverse_job.py and writes tests/golden/noise_inverse.npz
 (inverted latent, combined noise, per mode).  The gpu test replays the same job on our delegate with the real kernels.
-Usage: python -m oracle.make_noise_inverse_golden
+Usage: TD_REFERENCE_ROOT=<checkout of the original extension> python -m oracle.make_noise_inverse_golden
 """
 import os
 import sys
@@ -19,7 +19,7 @@ def main():
     from oracle import ref_shim
     import noise_inverse_job as job
     if not ref_shim.available():
-        sys.exit("reference tree not present")
+        sys.exit("reference tree not found: set TD_REFERENCE_ROOT to a checkout of the original extension")
     ref = ref_shim.load()
     out = {}
     for mode in job.MODES:

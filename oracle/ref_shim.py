@@ -1,16 +1,16 @@
 """TEST INFRASTRUCTURE ONLY -- stub A1111 host so the UNMODIFIED reference imports.
 
-The reference (`/root/reference`, read-only, CC BY-NC-SA) is a WebUI extension whose
+The reference (the original extension, CC BY-NC-SA) is a WebUI extension whose
 modules import `modules.*` (A1111), `ldm`, `k_diffusion` and `gradio` at import time
 (tile_utils/utils.py:11-14, tile_utils/typing.py:6-29, scripts/tilevae.py:60-70,
-tile_utils/attn.py:8-10).  None of those exist here.  This shim injects empty
-`types.ModuleType` stand-ins for exactly the names those import lines need, puts
-`/root/reference` on `sys.path`, and returns the reference's own modules so that
-`oracle/make_golden.py` and the CPU tests can call the reference's real code.
-
-It only works where `/root/reference` exists (the build container).  Nothing on
-the GPU box may import it: `available()` is the guard.  No reference source is
-copied; this file contains only stubs.
+tile_utils/attn.py:8-10).  None of those exist here.  `install()` injects empty
+`types.ModuleType` stand-ins for exactly the names those import lines need (plus a
+deterministic prompt parser); the CPU tests run our delegate under that stub host.
+`load()` additionally puts the reference checkout named by $TD_REFERENCE_ROOT on
+`sys.path` and returns the reference's own modules, so that the fixture generators
+(`oracle/make_*.py`) can call the reference's real code.  No test needs the
+reference: they compare with what those generators stored under tests/golden/.
+No reference source is copied; this file contains only stubs.
 """
 from __future__ import annotations
 
@@ -19,11 +19,11 @@ import os
 import sys
 import types
 
-REFERENCE_ROOT = os.environ.get("TD_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("TD_REFERENCE_ROOT", "")
 
 
 def available() -> bool:
-    return os.path.isfile(os.path.join(REFERENCE_ROOT, "tile_methods", "multidiffusion.py"))
+    return bool(REFERENCE_ROOT) and os.path.isfile(os.path.join(REFERENCE_ROOT, "tile_methods", "multidiffusion.py"))
 
 
 class _State:
@@ -45,11 +45,15 @@ class _CmdOpts:
     md_max_regions = 8
 
 
+_created = []
+
+
 def _mod(name: str, **attrs) -> types.ModuleType:
     m = sys.modules.get(name)
     if m is None:
         m = types.ModuleType(name)
         sys.modules[name] = m
+        _created.append(name)
         parent, _, child = name.rpartition(".")
         if parent:
             setattr(_mod(parent), child, m)
@@ -97,16 +101,20 @@ def fake_reconstruct_cond(cond, step):
 _installed = False
 
 
-def install(device: str = "cpu"):
-    """Inject the stub host.  Idempotent."""
+def _host() -> types.SimpleNamespace:
+    return types.SimpleNamespace(shared=sys.modules["modules.shared"], devices=sys.modules["modules.devices"],
+                                 KDiffusionSampler=sys.modules["modules.sd_samplers_kdiffusion"].KDiffusionSampler,
+                                 CompVisSampler=sys.modules["modules.sd_samplers_timesteps"].CompVisSampler)
+
+
+def install(device: str = "cpu") -> types.SimpleNamespace:
+    """Inject the stub host (needs no reference) and return its `shared`, `devices` and sampler classes.  Idempotent."""
     global _installed
     import torch
 
     if _installed:
         sys.modules["modules.devices"].device = torch.device(device)
-        return
-    if not available():
-        raise RuntimeError(f"reference tree not found at {REFERENCE_ROOT}")
+        return _host()
 
     class KDiffusionSampler:  # isinstance() target, abstractdiffusion.py:77-79
         pass
@@ -177,18 +185,28 @@ def install(device: str = "cpu"):
     _mod("ldm.modules")
     _mod("ldm.modules.diffusionmodules")
     _mod("ldm.modules.diffusionmodules.model", AttnBlock=_Dummy, MemoryEfficientAttnBlock=_Dummy)
-
-    if REFERENCE_ROOT not in sys.path:
-        sys.path.insert(0, REFERENCE_ROOT)
     _installed = True
+    return _host()
+
+
+def uninstall() -> None:
+    """Drop the stand-in modules `install()` created, so that code run afterwards sees no WebUI."""
+    global _installed
+    for name in reversed(_created):
+        sys.modules.pop(name, None)
+    _created.clear()
+    _installed = False
 
 
 def load(device: str = "cpu"):
-    """Return a namespace of the reference's own (unmodified) modules."""
-    install(device)
+    """Return the stub host of `install()` plus the reference's own (unmodified) modules."""
+    if not available():
+        raise RuntimeError("reference tree not found: set TD_REFERENCE_ROOT to a checkout of the original extension")
+    ns = install(device)
+    if REFERENCE_ROOT not in sys.path:
+        sys.path.insert(0, REFERENCE_ROOT)
     import importlib
 
-    ns = types.SimpleNamespace()
     ns.utils = importlib.import_module("tile_utils.utils")
     ns.abstractdiffusion = importlib.import_module("tile_methods.abstractdiffusion")
     ns.multidiffusion = importlib.import_module("tile_methods.multidiffusion")
@@ -196,10 +214,6 @@ def load(device: str = "cpu"):
     ns.demofusion = importlib.import_module("tile_methods.demofusion")
     ns.tilevae = importlib.import_module("scripts.tilevae")
     ns.attn = importlib.import_module("tile_utils.attn")
-    ns.shared = sys.modules["modules.shared"]
-    ns.devices = sys.modules["modules.devices"]
-    ns.KDiffusionSampler = sys.modules["modules.sd_samplers_kdiffusion"].KDiffusionSampler
-    ns.CompVisSampler = sys.modules["modules.sd_samplers_timesteps"].CompVisSampler
     return ns
 
 
@@ -213,7 +227,7 @@ def make_p(width: int, height: int, sampler_name: str = "Euler a"):
 def make_kdiff_sampler(inner_forward):
     """Fake k-diffusion sampler: `.model_wrap_cfg.inner_model.forward` is what
     MultiDiffusion.hook patches (multidiffusion.py:22-23)."""
-    ref = load()
+    ref = install()
 
     class _Sampler(ref.KDiffusionSampler):
         pass

@@ -1,10 +1,55 @@
 """Shared helpers for the parity tests (bit views, oracle plans)."""
+import contextlib
 import hashlib
+import os
 
 import numpy as np
 import torch
 
 DTYPES = {"f16": torch.float16, "bf16": torch.bfloat16, "f32": torch.float32}
+REFERENCE_TRACES = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_traces.npz")
+
+
+def digest(t: torch.Tensor) -> int:
+    """First 8 bytes of the sha256 of a tensor's dtype, shape and bit pattern: what tests/golden/reference_traces.npz
+    (oracle/make_reference_traces.py) keeps of every tensor the reference handed out.  Some traces start from seeded
+    `torch.randn` draws, which are the same on every host where ATen runs its AVX2 or AVX-512 kernels."""
+    t = t.detach().cpu().contiguous()
+    h = hashlib.sha256(f"{t.dtype}{tuple(t.shape)}".encode())
+    h.update(t.reshape(-1).view(torch.uint8).numpy().tobytes())
+    return int.from_bytes(h.digest()[:8], "little")
+
+
+def reference_trace(key: str):
+    """The stored reference trace `key` (uint64 digests, int32 boxes or a string), or None if the reference has none."""
+    with np.load(REFERENCE_TRACES) as g:
+        return g[key] if key in g.files else None
+
+
+def assert_trace(got, key: str):
+    """`got`: digests of our tensors, in the order the reference's were recorded under `key`."""
+    want = reference_trace(key)
+    assert want is not None, f"{key}: no reference trace stored (oracle/make_reference_traces.py)"
+    want = [int(v) for v in want]
+    assert len(got) == len(want), f"{key}: {len(got)} tensors vs the reference's {len(want)}"
+    bad = [i for i, (a, b) in enumerate(zip(got, want)) if a != b]
+    assert not bad, f"{key}: tensors {bad} (of {len(want)}) differ from the reference's"
+
+
+@contextlib.contextmanager
+def stub_webui(monkeypatch):
+    """Our delegate under the stub WebUI the reference traces were recorded in (oracle/ref_shim.py: `modules.*`
+    stand-ins, deterministic prompt parser), with its buffers on the host as on a machine without a GPU."""
+    from multidiffusion_upscaler_for_automatic1111_b200 import host
+    from oracle import ref_shim
+    ns = ref_shim.install()
+    host._a1111_cache.clear()
+    monkeypatch.setattr(host, "device", lambda: torch.device("cpu"))
+    try:
+        yield ns
+    finally:
+        ref_shim.uninstall()
+        host._a1111_cache.clear()
 
 
 def bits(t: torch.Tensor) -> np.ndarray:

@@ -7,7 +7,7 @@ import numpy as np
 import pytest
 import torch
 
-from helpers import DTYPES, bits
+from helpers import DTYPES, assert_trace, bits, digest, stub_webui
 from oracle import demofusion as odf
 from oracle import synth, tiling
 from oracle.make_golden import DEMO_CASES, DEMO_CFG, demo_denoise
@@ -193,54 +193,59 @@ def test_jitter_oracle_and_windows_match_reference_fixture(golden_dir):
         assert [d.tile_bs, d.global_tile_bs, d.global_num_tiles, d.jitter_range] == list(g[name + "_sizes"])
 
 
-def test_forward_one_step_pads_and_crops_like_the_reference():
-    """forward_one_step (demofusion.py:185-214): skip-residual mix, zero-pad by jitter_range, CFG forward with the tiled
-    step patched in, crop back.  Live reference next to our delegate on CPU, the tiled step itself replaced by a stub."""
+def _forward_one_step(webui, cls):
+    """forward_one_step (demofusion.py:185-214) of a `cls` delegate with the tiled step itself replaced by a stub: checks
+    the zero padding the stub sees and returns the cropped CFG output."""
     import random
-    from oracle import ref_shim
-    if not ref_shim.available():
-        pytest.skip("reference tree not present")
-    from multidiffusion_upscaler_for_automatic1111_b200 import DemoFusion, host
     from oracle.make_golden import DEMO_JITTER_SEED
-    ref = ref_shim.load()
-    host._a1111_cache.clear()
     c = DEMO_CFG
     g = torch.Generator().manual_seed(1)
     x = torch.randn(c["N"], c["C"], c["H"], c["W"], generator=g)
     px, pn = torch.randn(x.shape, generator=g), torch.randn(x.shape, generator=g)
-    outs = []
-    for cls in (ref.demofusion.DemoFusion, DemoFusion):
-        p = _jitter_p(True)
-        p.x, p.noise, p.disable_extra_networks, p.batch_size = px, pn, True, 1
-        seen = {}
+    p = _jitter_p(True)
+    p.x, p.noise, p.disable_extra_networks, p.batch_size = px, pn, True, 1
+    seen = {}
 
-        def forward_ori(x_in, sigma, **kw):
-            return cfg.inner_model.forward(x_in, sigma, kw.get("cond"))
-        inner = types.SimpleNamespace(forward="original")
-        cfg = types.SimpleNamespace(inner_model=inner, image_cfg_scale=None, forward=forward_ori, step=0)
+    def forward_ori(x_in, sigma, **kw):
+        return cfg.inner_model.forward(x_in, sigma, kw.get("cond"))
+    inner = types.SimpleNamespace(forward="original")
+    cfg = types.SimpleNamespace(inner_model=inner, image_cfg_scale=None, forward=forward_ori, step=0)
 
-        class _S(ref.KDiffusionSampler):
-            pass
-        sampler = _S()
-        sampler.model_wrap_cfg = cfg
-        d = cls(p, sampler)
-        d.window_size, d.sig = c["window"], c["sig"]
-        random.seed(DEMO_JITTER_SEED)
-        d.get_views(c["overlap"], c["tile_bs"], c["tile_bs_g"])
-        d.hook()
+    class _S(webui.KDiffusionSampler):
+        pass
+    sampler = _S()
+    sampler.model_wrap_cfg = cfg
+    d = cls(p, sampler)
+    d.window_size, d.sig = c["window"], c["sig"]
+    random.seed(DEMO_JITTER_SEED)
+    d.get_views(c["overlap"], c["tile_bs"], c["tile_bs_g"])
+    d.hook()
 
-        def fake_step(x_in, sigma, cond, seen=seen):
-            seen["shape"] = tuple(x_in.shape)
-            seen["border"] = float(x_in[:, :, :d.jitter_range].abs().max())
-            return x_in * 2 + 1
-        d.sample_one_step = fake_step
-        out = cfg.forward(x, torch.full((c["N"],), 3.0), cond=None)
-        assert cfg.inner_model.forward == "original"                 # restored after the call
-        jr = d.jitter_range
-        assert jr == 6 and seen["shape"] == (c["N"], c["C"], c["H"] + 2 * jr, c["W"] + 2 * jr) and seen["border"] == 0.0
-        outs.append(out)
-    assert outs[0].shape == x.shape and torch.equal(outs[0], outs[1])
-    host._a1111_cache.clear()
+    def fake_step(x_in, sigma, cond, seen=seen):
+        seen["shape"] = tuple(x_in.shape)
+        seen["border"] = float(x_in[:, :, :d.jitter_range].abs().max())
+        return x_in * 2 + 1
+    d.sample_one_step = fake_step
+    out = cfg.forward(x, torch.full((c["N"],), 3.0), cond=None)
+    assert cfg.inner_model.forward == "original"                 # restored after the call
+    jr = d.jitter_range
+    assert jr == 6 and seen["shape"] == (c["N"], c["C"], c["H"] + 2 * jr, c["W"] + 2 * jr) and seen["border"] == 0.0
+    assert out.shape == x.shape
+    return out
+
+
+def reference_traces(ref):
+    """The reference's side of test_forward_one_step_pads_and_crops_like_the_reference (oracle/make_reference_traces.py)."""
+    return {"demofusion_forward_one_step": [digest(_forward_one_step(ref, ref.demofusion.DemoFusion))]}
+
+
+def test_forward_one_step_pads_and_crops_like_the_reference(monkeypatch):
+    """Skip-residual mix, zero-pad by jitter_range, CFG forward with the tiled step patched in, crop back: our delegate on
+    CPU under the stub WebUI against the reference's output under the same stub (tests/golden/reference_traces.npz)."""
+    from multidiffusion_upscaler_for_automatic1111_b200 import DemoFusion
+    with stub_webui(monkeypatch) as webui:
+        out = _forward_one_step(webui, DemoFusion)
+    assert_trace([digest(out)], "demofusion_forward_one_step")
 
 
 # ------------------------------------------------------------------------------------------ delegate host logic on CPU

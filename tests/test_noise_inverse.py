@@ -1,8 +1,9 @@
 """Tiled noise inversion (SURVEY.md section 8(f)-3): `init_noise_inverse` replaces the sampler's `sample_img2img`; the
 Euler inversion loop runs the tiled denoiser (`get_noise`), the result is mixed with fresh noise under the retouch mask.
 
-The UNMODIFIED reference (oracle/ref_shim.py) runs next to our delegate on CPU, with the device kernels swapped for the
-oracle's scatter / blend (pinned by tests/test_gpu_diffusion.py); outputs must be identical.
+Our delegate runs on CPU under the stub WebUI of oracle/ref_shim.py, with the device kernels swapped for the oracle's
+scatter / blend (pinned by tests/test_gpu_diffusion.py); its outputs must be identical to those of the UNMODIFIED
+reference under the same stub (`reference_traces` below, stored in tests/golden/reference_traces.npz).
 """
 import types
 
@@ -10,9 +11,8 @@ import numpy as np
 import pytest
 import torch
 
-from oracle import blend, ref_shim
-
-pytestmark = pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present")
+from helpers import assert_trace, digest, reference_trace, stub_webui
+from oracle import blend
 
 W, H = 64, 48
 ROWS = [(True, 0.1, 0.2, 0.5, 0.4, "a cat", "", "Background", 0.2, -1),
@@ -40,7 +40,7 @@ def _image():
     return Image.fromarray(a)
 
 
-def _job(ref, cls, settings, draw_background, with_regions):
+def _job(ref, cls, settings, draw_background, with_regions, cache_type):
     """(delegate, sampler, p, cache) ready for sampler.sample_img2img(...)."""
     sd_model = types.SimpleNamespace(sd_model_hash="abc", get_learned_conditioning=lambda prompts: torch.full((len(prompts), 77, 8), 0.25))
     g = torch.Generator().manual_seed(5)
@@ -64,7 +64,7 @@ def _job(ref, cls, settings, draw_background, with_regions):
 
     def set_cache(x0, xt, prompts):
         cache["sets"] += 1
-        cache["v"] = ref.utils.NoiseInverseCache("abc", x0, xt, 4, 1.5, prompts)
+        cache["v"] = cache_type("abc", x0, xt, 4, 1.5, prompts)
 
     d = cls(p, sampler)
     d.init_grid_bbox(16, 16, 8, 4)
@@ -101,35 +101,46 @@ def _oracle_engine(monkeypatch):
     monkeypatch.setattr(abstractdiffusion.AbstractDiffusion, "_check_input", lambda self, x: x.contiguous())
 
 
-@pytest.mark.parametrize("mode", ["grid", "grid+regions", "regions_only"])
-def test_noise_inversion_like_the_reference(monkeypatch, mode):
-    from multidiffusion_upscaler_for_automatic1111_b200 import MultiDiffusion, host
-    ref = ref_shim.load()
-    host._a1111_cache.clear()
-    _oracle_engine(monkeypatch)
-    ref.shared.sd_model.apply_model = lambda x, t, cond=None: x * 0.5 + t.view(-1, 1, 1, 1) * 1e-3 + cond["c_crossattn"][0].mean() * 0.1
-    if hasattr(ref.shared.sd_model, "apply_model_original_md"):
-        del ref.shared.sd_model.apply_model_original_md
-    with_regions, bg = mode != "grid", mode != "regions_only"
+MODES = ["grid", "grid+regions", "regions_only"]
 
+
+def _invert(webui, cls, settings, cache_type, mode):
+    """Two img2img starts of the same job, the second one served from the cache: digests of the inverted latent and of
+    both combined noises, and the step count handed to the sampler."""
     # region prompts at a noise-inversion step go through the (stand-in) prompt parser: [tokens] -> unsqueeze -> apply_model
+    webui.shared.sd_model.apply_model = lambda x, t, cond=None: x * 0.5 + t.view(-1, 1, 1, 1) * 1e-3 + cond["c_crossattn"][0].mean() * 0.1
+    if hasattr(webui.shared.sd_model, "apply_model_original_md"):
+        del webui.shared.sd_model.apply_model_original_md
+    webui.shared.state.sampling_step = 0
+    with_regions, bg = mode != "grid", mode != "regions_only"
     noise = torch.randn(1, 4, H, W, generator=torch.Generator().manual_seed(9))
     x = torch.zeros(1, 4, H, W)
-    results = []
-    for cls, settings in ((ref.multidiffusion.MultiDiffusion, {i: ref.utils.BBoxSettings(*r) for i, r in enumerate(ROWS)}),
-                          (MultiDiffusion, {i: r for i, r in enumerate(ROWS)})):
-        ref.shared.state.sampling_step = 0
-        d, sampler, p, cache = _job(ref, cls, settings, bg, with_regions)
-        assert sampler.sample_img2img.__func__ is not None          # replaced by a bound method of the sampler
-        first = sampler.sample_img2img(p, x, noise, None, None)
-        assert cache["sets"] == 1
-        second = sampler.sample_img2img(p, x, noise, None, None)     # cache hit: no second inversion
-        assert cache["sets"] == 1
-        results.append((first, second, cache["v"].xt))
-    (rf, rs, rxt), (of, os_, oxt) = results
-    assert of[0] == rf[0] == "sampled" and of[3] == rf[3]
-    assert torch.equal(oxt, rxt), "inverted latent"
-    assert torch.equal(of[2], rf[2]), "combined noise"
-    assert torch.equal(os_[2], rs[2]), "combined noise from the cache"
-    assert torch.isfinite(of[2]).all() and not torch.equal(of[2], noise)
-    host._a1111_cache.clear()
+    d, sampler, p, cache = _job(webui, cls, settings, bg, with_regions, cache_type)
+    assert sampler.sample_img2img.__func__ is not None          # replaced by a bound method of the sampler
+    first = sampler.sample_img2img(p, x, noise, None, None)
+    assert cache["sets"] == 1
+    second = sampler.sample_img2img(p, x, noise, None, None)     # cache hit: no second inversion
+    assert cache["sets"] == 1
+    assert first[0] == second[0] == "sampled"
+    assert torch.isfinite(first[2]).all() and not torch.equal(first[2], noise)
+    return [digest(cache["v"].xt), digest(first[2]), digest(second[2])], str(first[3])
+
+
+def reference_traces(ref):
+    """The reference's side of the test below (oracle/make_reference_traces.py)."""
+    out = {}
+    for mode in MODES:
+        out[f"noise_inverse_{mode}"], out[f"noise_inverse_{mode}_steps"] = _invert(
+            ref, ref.multidiffusion.MultiDiffusion, {i: ref.utils.BBoxSettings(*r) for i, r in enumerate(ROWS)}, ref.utils.NoiseInverseCache, mode)
+    return out
+
+
+@pytest.mark.parametrize("mode", MODES)
+def test_noise_inversion_like_the_reference(monkeypatch, mode):
+    from multidiffusion_upscaler_for_automatic1111_b200 import MultiDiffusion
+    from multidiffusion_upscaler_for_automatic1111_b200.tile_utils import utils
+    with stub_webui(monkeypatch) as webui:
+        _oracle_engine(monkeypatch)
+        trace, steps = _invert(webui, MultiDiffusion, {i: r for i, r in enumerate(ROWS)}, utils.NoiseInverseCache, mode)
+    assert steps == str(reference_trace(f"noise_inverse_{mode}_steps"))
+    assert_trace(trace, f"noise_inverse_{mode}")

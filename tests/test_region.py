@@ -117,8 +117,9 @@ def test_oracle_region_step_matches_reference_fixture(gold, case, method, dn):
 
 # ------------------------------------------------------------------------------------------------ delegates
 def _oracle_engine(monkeypatch):
-    """Swap the three device entry points for the oracle so the delegates' host logic runs on CPU tensors."""
-    from multidiffusion_upscaler_for_automatic1111_b200 import engine
+    """Swap the three device entry points for the oracle so the delegates' host logic runs on CPU tensors (their
+    buffers too, also where a GPU is present)."""
+    from multidiffusion_upscaler_for_automatic1111_b200 import engine, host
     from multidiffusion_upscaler_for_automatic1111_b200.tile_methods import abstractdiffusion
 
     def bbs(g):
@@ -144,6 +145,7 @@ def _oracle_engine(monkeypatch):
     monkeypatch.setattr(engine, "blend_multidiffusion", blend_multidiffusion)
     monkeypatch.setattr(engine, "blend_mixture", blend_mixture)
     monkeypatch.setattr(abstractdiffusion.AbstractDiffusion, "_check_input", lambda self, x: x.contiguous())
+    monkeypatch.setattr(host, "device", lambda: torch.device("cpu"))
 
 
 def _run_delegate(method, x, bg, rows, device):

@@ -1,8 +1,9 @@
 """ControlNet / StableSR tile caches (SURVEY.md section 8(f)-2): the per-batch hint tiles our delegate caches and
 hands to the extension objects must equal the reference's, for k-diffusion and DDIM samplers, grid and custom bboxes.
 
-CPU: the UNMODIFIED reference (oracle/ref_shim.py) next to our delegate, with the scatter kernel swapped for the
-oracle's scatter (the kernel itself is pinned by tests/test_gpu_diffusion.py).  GPU: the same caches through
+CPU: our delegate under the stub WebUI of oracle/ref_shim.py, with the scatter kernel swapped for the oracle's scatter
+(the kernel itself is pinned by tests/test_gpu_diffusion.py), against what the UNMODIFIED reference cached under the
+same stub (`reference_traces` below, stored in tests/golden/reference_traces.npz).  GPU: the same caches through
 td_scatter_tiles on the x8-scaled tile plan, against plain slicing.
 """
 import types
@@ -10,6 +11,7 @@ import types
 import pytest
 import torch
 
+from helpers import assert_trace, digest, stub_webui
 from oracle import blend, ref_shim
 
 W, H = 64, 48
@@ -50,99 +52,104 @@ def _delegate(cls, sampler, settings, with_regions):
     return d
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present")
+def _sampler(webui, kdiff):
+    if kdiff:
+        return ref_shim.make_kdiff_sampler(lambda x, s, cond=None: x)
+
+    class _S(webui.CompVisSampler):
+        pass
+    s = _S()
+    s.model_wrap_cfg = types.SimpleNamespace(inner_model=types.SimpleNamespace(forward=None), image_cfg_scale=None, step=0)
+    return s
+
+
+def _controlnet_trace(d, cs, tensor_cpu, with_regions):
+    """Digests of the hint tiles `d` caches for the ControlNet units of `cs`, then of the hints it hands them at the first
+    and last batch (condition / denoise), at a custom region and after the reset."""
+    d.init_controlnet(cs, tensor_cpu)
+    d.init_done()
+    if getattr(d, "pbar", None) is not None:
+        d.pbar.disable = True
+    hints = lambda: [digest(u.hint_cond) for u in cs.latest_network.control_params]
+    out = [digest(t) for per_unit in d.control_tensor_batch for t in per_unit]
+    if with_regions:
+        out += [digest(t) for per_unit in d.control_tensor_custom for t in per_unit]
+    for batch_id in (0, d.num_batches - 1):
+        n_tiles = len(d.batched_bboxes[batch_id])
+        for is_denoise in (False, True):
+            d.switch_controlnet_tensors(batch_id, 2, n_tiles, is_denoise=is_denoise)
+            out += hints()
+    if with_regions:
+        d.set_custom_controlnet_tensors(1, 3)
+        out += hints()
+    d.reset_controlnet_tensors()
+    return out + hints()
+
+
+def _stablesr_trace(d, latent):
+    """Digests of the latent tiles `d` caches for StableSR, then of the latent it hands the model per batch and at a
+    custom region; after the reset the model must hold the caller's latent again."""
+    model = types.SimpleNamespace(set_image_hooks={}, latent_image=None)
+    d.init_stablesr(types.SimpleNamespace(stablesr_model=model))
+    d.init_done()
+    if getattr(d, "pbar", None) is not None:
+        d.pbar.disable = True
+    model.set_image_hooks["TiledDiffusion"](latent)
+    out = [digest(t) for t in d.stablesr_tensor_batch]
+    for b in range(d.num_batches):
+        d.switch_stablesr_tensors(b)
+        out.append(digest(model.latent_image))
+    d.set_custom_stablesr_tensors(1)
+    out.append(digest(model.latent_image))
+    d.reset_stablesr_tensors()
+    assert model.latent_image is latent
+    return out
+
+
+CONTROLNET_CASES = [(kdiff, with_regions, tensor_cpu) for kdiff in (True, False) for with_regions in (False, True) for tensor_cpu in (False, True)]
+
+
+def _latent():
+    return torch.arange(2 * 4 * H * W, dtype=torch.float32).view(2, 4, H, W)
+
+
+def reference_traces(ref):
+    """The reference's side of the tests below (oracle/make_reference_traces.py)."""
+    out = {}
+    settings = {i: ref.utils.BBoxSettings(*r) for i, r in enumerate(ROWS)}
+    for kdiff, with_regions, tensor_cpu in CONTROLNET_CASES:
+        d = _delegate(ref.multidiffusion.MultiDiffusion, _sampler(ref, kdiff), settings, with_regions)
+        assert d.is_kdiff == kdiff
+        out[f"controlnet_{kdiff}_{with_regions}_{tensor_cpu}"] = _controlnet_trace(d, _controlnet_script(), tensor_cpu, with_regions)
+    d = _delegate(ref.multidiffusion.MultiDiffusion, ref_shim.make_kdiff_sampler(lambda x, s, cond=None: x), settings, True)
+    out["stablesr"] = _stablesr_trace(d, _latent())
+    return out
+
+
 @pytest.mark.parametrize("kdiff", [True, False], ids=["kdiff", "ddim"])
 @pytest.mark.parametrize("with_regions", [False, True], ids=["grid", "grid+regions"])
 @pytest.mark.parametrize("tensor_cpu", [False, True], ids=["dev", "cpu_cache"])
 def test_controlnet_tile_caches_like_the_reference(monkeypatch, kdiff, with_regions, tensor_cpu):
-    from multidiffusion_upscaler_for_automatic1111_b200 import MultiDiffusion, host
-    ref = ref_shim.load()
-    host._a1111_cache.clear()
-    _oracle_scatter(monkeypatch)
-
-    def sampler():
-        if kdiff:
-            return ref_shim.make_kdiff_sampler(lambda x, s, cond=None: x)
-
-        class _S(ref.CompVisSampler):
-            pass
-        s = _S()
-        s.model_wrap_cfg = types.SimpleNamespace(inner_model=types.SimpleNamespace(forward=None), image_cfg_scale=None, step=0)
-        return s
-
-    d_ref = _delegate(ref.multidiffusion.MultiDiffusion, sampler(), {i: ref.utils.BBoxSettings(*r) for i, r in enumerate(ROWS)}, with_regions)
-    d_our = _delegate(MultiDiffusion, sampler(), {i: r for i, r in enumerate(ROWS)}, with_regions)
-    assert d_our.is_kdiff == kdiff == d_ref.is_kdiff
-    scripts = []
-    for d in (d_ref, d_our):
+    from multidiffusion_upscaler_for_automatic1111_b200 import MultiDiffusion
+    with stub_webui(monkeypatch) as webui:
+        _oracle_scatter(monkeypatch)
+        d = _delegate(MultiDiffusion, _sampler(webui, kdiff), {i: r for i, r in enumerate(ROWS)}, with_regions)
+        assert d.is_kdiff == kdiff
         cs = _controlnet_script()
-        scripts.append(cs)
-        d.init_controlnet(cs, tensor_cpu)
-        d.init_done()
-        if getattr(d, "pbar", None) is not None:
-            d.pbar.disable = True
-    cs_ref, cs_our = scripts
-
-    assert len(d_our.control_tensor_batch) == len(d_ref.control_tensor_batch) == 2
-    for pr, po in zip(d_ref.control_tensor_batch, d_our.control_tensor_batch):
-        assert len(pr) == len(po) == d_ref.num_batches
-        for tr, to in zip(pr, po):
-            assert tr.shape == to.shape and torch.equal(tr, to)
-    if with_regions:
-        for pr, po in zip(d_ref.control_tensor_custom, d_our.control_tensor_custom):
-            for tr, to in zip(pr, po):
-                assert torch.equal(tr, to)
-
-    for batch_id in (0, d_ref.num_batches - 1):
-        n_tiles = len(d_ref.batched_bboxes[batch_id])
-        for is_denoise in (False, True):
-            for d in (d_ref, d_our):
-                d.switch_controlnet_tensors(batch_id, 2, n_tiles, is_denoise=is_denoise)
-            for a, b in zip(cs_ref.latest_network.control_params, cs_our.latest_network.control_params):
-                assert a.hint_cond.shape == b.hint_cond.shape and torch.equal(a.hint_cond, b.hint_cond)
-    if with_regions:
-        for d in (d_ref, d_our):
-            d.set_custom_controlnet_tensors(1, 3)
-        for a, b in zip(cs_ref.latest_network.control_params, cs_our.latest_network.control_params):
-            assert torch.equal(a.hint_cond, b.hint_cond)
-    for d in (d_ref, d_our):
-        d.reset_controlnet_tensors()
-    for a, b in zip(cs_ref.latest_network.control_params, cs_our.latest_network.control_params):
-        assert a.hint_cond.shape == (1, 3, H * 8, W * 8) and torch.equal(a.hint_cond, b.hint_cond)
-    host._a1111_cache.clear()
+        trace = _controlnet_trace(d, cs, tensor_cpu, with_regions)
+    assert len(d.control_tensor_batch) == 2 and all(len(per_unit) == d.num_batches for per_unit in d.control_tensor_batch)
+    assert all(u.hint_cond.shape == (1, 3, H * 8, W * 8) for u in cs.latest_network.control_params)
+    assert_trace(trace, f"controlnet_{kdiff}_{with_regions}_{tensor_cpu}")
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present")
 def test_stablesr_tile_caches_like_the_reference(monkeypatch):
-    from multidiffusion_upscaler_for_automatic1111_b200 import MultiDiffusion, host
-    ref = ref_shim.load()
-    host._a1111_cache.clear()
-    _oracle_scatter(monkeypatch)
-    latent = torch.arange(2 * 4 * H * W, dtype=torch.float32).view(2, 4, H, W)
-    models = []
-    for cls, settings in ((ref.multidiffusion.MultiDiffusion, {i: ref.utils.BBoxSettings(*r) for i, r in enumerate(ROWS)}),
-                          (MultiDiffusion, {i: r for i, r in enumerate(ROWS)})):
-        d = _delegate(cls, ref_shim.make_kdiff_sampler(lambda x, s, cond=None: x), settings, True)
-        model = types.SimpleNamespace(set_image_hooks={}, latent_image=None)
-        d.init_stablesr(types.SimpleNamespace(stablesr_model=model))
-        d.init_done()
-        if getattr(d, "pbar", None) is not None:
-            d.pbar.disable = True
-        model.set_image_hooks["TiledDiffusion"](latent)
-        models.append((d, model))
-    (d_ref, m_ref), (d_our, m_our) = models
-    assert d_our.enable_stablesr and len(d_our.stablesr_tensor_batch) == len(d_ref.stablesr_tensor_batch)
-    for b in range(d_ref.num_batches):
-        for d in (d_ref, d_our):
-            d.switch_stablesr_tensors(b)
-        assert m_ref.latent_image.shape == m_our.latent_image.shape and torch.equal(m_ref.latent_image, m_our.latent_image)
-    for d in (d_ref, d_our):
-        d.set_custom_stablesr_tensors(1)
-    assert torch.equal(m_ref.latent_image, m_our.latent_image)
-    for d in (d_ref, d_our):
-        d.reset_stablesr_tensors()
-    assert m_our.latent_image is latent and m_ref.latent_image is latent
-    host._a1111_cache.clear()
+    from multidiffusion_upscaler_for_automatic1111_b200 import MultiDiffusion
+    with stub_webui(monkeypatch):
+        _oracle_scatter(monkeypatch)
+        d = _delegate(MultiDiffusion, ref_shim.make_kdiff_sampler(lambda x, s, cond=None: x), {i: r for i, r in enumerate(ROWS)}, True)
+        trace = _stablesr_trace(d, _latent())
+    assert d.enable_stablesr
+    assert_trace(trace, "stablesr")
 
 
 def test_scaled_grid_is_the_tile_plan_times_opt_f():
